@@ -2,7 +2,7 @@
 """
 bench.py -- GP posteriors/s at N=16384 (BASELINE.json metric) on N GPUs of one node.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   (N > 1: launched by torchrun, one rank per GPU; ranks process independent posterior draws -- the
    path's natural sharding, SURVEY.md section 8e "draw-parallel" -- so scaling is weak and there is no
    data-path collective; torch.distributed is used only for the barrier and the max-over-ranks.)
@@ -21,6 +21,9 @@ Gram(k_XX) -> N x N Cholesky -> Gram(k_pX) -> triangular solves -> posterior mea
           fp64 DMMA kernel on the same launch
   cpu_baseline  the oracle's restatement of the reference formulation (explicit inverse,
           oracle.exact_posterior) timed on the host cores on a bounded sample
+
+--dump-outputs DIR writes what the last timed step returned, mean.npy and var.npy ([S, P] float64), so that two builds
+can be compared output for output: the inputs depend only on the seed, the rank and --draws.
 """
 import argparse
 import json
@@ -238,6 +241,23 @@ def cpu_baseline(budget_s=30.0):
             "best_cpu_formulation": {"value": best["value"], "unit": "posteriors/s", "sample": best["sample"]}}
 
 
+DUMP_LIMIT_BYTES = 63 * 10 ** 6        # 64 MB less room for the .npy headers
+
+
+def dump_outputs(out_dir, arrays, suffix=""):
+    """Write each [S, P] array as out_dir/<name><suffix>.npy.  Above DUMP_LIMIT_BYTES in all, the same seeded sample of
+    draws (rows) is kept from every array and its row indices go to draws<suffix>.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    S = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(a[0].nbytes for a in arrays.values()) + 8          # + the row's index in draws.npy
+    keep = min(S, DUMP_LIMIT_BYTES // row_bytes)
+    if keep < S:
+        rows = np.sort(np.random.default_rng(0).choice(S, keep, replace=False))
+        arrays = dict({k: a[rows] for k, a in arrays.items()}, draws=rows.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
+
+
 def dist_workloads(ctx, ffi, rank, world, local, td, steps=3):
     """The two BASELINE configs whose data path has a real exchange step (SURVEY.md section 8e), run inside libb200gp.so over
     NCCL (gpax_b200/csrc/dist.cuh) -- STRONG scaling, reported as extra objects of the bench line:
@@ -370,7 +390,11 @@ def main():
     ap.add_argument("--draws", type=int, default=None, help="posterior draws per step (default 8)")
     ap.add_argument("--no-dist", action="store_true", help="skip the c4 / c5 exchange-step workloads")
     ap.add_argument("--opt", action="append", default=[], help="library option key=value (experiments)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's mean and var to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     if args.impl == "reference":
         run_reference_arm(args, int(os.environ.get("RANK", "0")))
@@ -422,6 +446,10 @@ def main():
     barrier_sync(td, local)
     t1 = time.perf_counter()
     clocks = sampler.stop(t0, t1)
+    if args.dump_outputs:
+        assert (info == 0).all(), f"factorisation failed in the last timed step: info={info}"
+        dump_outputs(args.dump_outputs, {"mean": dmean.download(), "var": dvar.download()},
+                     f"_rank{rank}" if world > 1 else "")
     wall_ms = (t1 - t0) * 1e3
     dev_ms = max_over_ranks(td, local, dev_ms)
     wall_ms = max_over_ranks(td, local, wall_ms)

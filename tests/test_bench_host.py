@@ -56,3 +56,28 @@ def test_cpu_baseline_scales_by_measured_growth(monkeypatch):
     assert "N=4096" in out["best_cpu_formulation"]["sample"]
     assert abs(1.0 / out["best_cpu_formulation"]["value"] - 0.2 * 16) < 1e-9
     assert bench.WORKLOAD == small
+
+
+def test_dump_outputs_writes_all_or_a_seeded_sample(tmp_path, monkeypatch):
+    """--dump-outputs: every draw while the arrays fit the limit; above it the same seeded rows of each array, bounded"""
+    sys.path.insert(0, ROOT)
+    import bench
+    S, P = 40, 16
+    mean = np.arange(S * P, dtype=np.float64).reshape(S, P)
+    var = mean + 0.5
+    bench.dump_outputs(str(tmp_path / "all"), {"mean": mean, "var": var})
+    assert sorted(os.listdir(tmp_path / "all")) == ["mean.npy", "var.npy"]
+    np.testing.assert_array_equal(np.load(tmp_path / "all" / "mean.npy"), mean)
+    np.testing.assert_array_equal(np.load(tmp_path / "all" / "var.npy"), var)
+
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 10 * (2 * P * 8 + 8))        # room for 10 of the 40 draws
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), {"mean": mean, "var": var}, "_rank1")
+    assert sorted(os.listdir(tmp_path / "a")) == ["draws_rank1.npy", "mean_rank1.npy", "var_rank1.npy"]
+    rows = np.load(tmp_path / "a" / "draws_rank1.npy")
+    assert rows.dtype == np.float64 and rows.shape == (10,) and len(set(rows)) == 10
+    r = rows.astype(int)
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "mean_rank1.npy"), mean[r])
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "var_rank1.npy"), var[r])
+    np.testing.assert_array_equal(np.load(tmp_path / "b" / "draws_rank1.npy"), rows)
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= bench.DUMP_LIMIT_BYTES + 3 * 128
